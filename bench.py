@@ -61,7 +61,12 @@ def parse_args():
     ap.add_argument("--replicas", action="store_true", help="diagnostic: under torchrun every rank runs an INDEPENDENT single-rank "
                     "solution (no halo exchange); shows what N busy GPUs of one box cost before any exchange")
     ap.add_argument("--opt", action="append", default=[], help="engine option key=value")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the p(t) they computed "
+                    "to DIR/p.npy (see dump_outputs), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the B200 path computed; it does not apply to --impl reference")
+    return args
 
 
 # --------------------------------------------------------------------------------------------------
@@ -240,7 +245,7 @@ def main_reference(args):
     wall = time.time() - t0
     pts = size ** 3
     line = {"metric": f"GPoints/s, iso3dfd-16 fp32 {size}^3 per GPU", "value": cb["value"], "unit": "GPoints/s", "impl": "reference", "n_gpus": args.gpus,
-            "steps": args.steps, "warmup": args.warmup, "ms_per_step": pts / (cb["value"] * 1e9) * 1e3, "higher_is_better": True,
+            "steps": steps, "warmup": args.warmup, "ms_per_step": pts / (cb["value"] * 1e9) * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"iso3dfd radius 8 (16th order) fp32, {size}^3 points on the host CPU (reference OpenMP/AVX path)",
                        "steps_per_trial": steps, "wall_s": round(wall, 1)},
@@ -252,6 +257,31 @@ def main_reference(args):
 # --------------------------------------------------------------------------------------------------
 # B200 arm
 # --------------------------------------------------------------------------------------------------
+DUMP_SEED, DUMP_BYTES = 20240, 32 << 20
+
+
+def dump_outputs(out_dir, p, rank, world):
+    """Write what the timed run_solution() left in p at its last valid step -- the array its caller reads back -- as
+    out_dir/p.npy (out_dir/p.rank<r>.npy per rank when several ranks run): float32 [plane, y, z], y-z planes at x offsets
+    drawn once from DUMP_SEED within the rank's domain, as many as fit the rank's share of DUMP_BYTES (8 whole planes,
+    32 MiB, at 1024^3 on one GPU); where one plane exceeds that share, seeded y rows of one plane.
+    The bench's inputs are fixed hash fields, so the same arguments give the same planes and the same values."""
+    import numpy as np
+    tl = p.get_last_valid_step_index()
+    first, last = p.domain_box(tl)
+    nx, ny, nz = (b - a + 1 for a, b in zip(first[1:], last[1:]))
+    share = DUMP_BYTES // world
+    k = max(1, min(nx, share // (4 * ny * nz)))
+    rng = np.random.default_rng(DUMP_SEED)
+    xs = sorted(rng.choice(nx, size=k, replace=False).tolist())
+    ys = sorted(rng.choice(ny, size=min(ny, max(1, share // (4 * nz))), replace=False).tolist())
+    planes = [p.get_elements_in_slice([tl, first[1] + x] + first[2:], [tl, first[1] + x] + last[2:]).reshape(ny, nz) for x in xs]
+    if len(ys) < ny:
+        planes = [a[ys] for a in planes]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "p.npy" if world == 1 else f"p.rank{rank}.npy"), np.stack(planes).astype(np.float32))
+
+
 def halo_check(capi, dist, rank, world, local, N, opts, seed=77, steps=3):
     """Cross-device correctness of the halo exchange at the bench's own geometry: a fresh multi-rank run of `steps`
     steps from global hash data; every rank then recomputes the 8 planes on its side of each x interface with a
@@ -445,6 +475,8 @@ def main_b200(args):
     pts_per_gpu = N ** 3
     value = pts_per_gpu * world * K / dev_s / 1e9
     checksum = p.checksum(p.get_last_valid_step_index())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, p, rank, world)
 
     # ---- sustained: the same loop for >= 2 s (the part settles to its power-capped clock) ---------------
     sustained = None

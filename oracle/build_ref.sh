@@ -18,10 +18,15 @@
 #   REF_ALL=1: every solution the golden fixtures were generated from (~90 kernel builds, over an hour);
 #   REF_RADII=1: only iso3dfd at radius 1 and 2 (fixtures of the temporal tile), ~3 min.
 #
-# Outputs: oracle/_ref/yask/  the reference's own output tree (stays in the build container);
-#          oracle/_ref/ship/  the few binaries the GPU box runs (copied from the tree; travels with gpurun);
-#          tools/_refc/       the reference's stencil COMPILER, which the product's build-time CUDA emitter
-#                             (yask_b200/emitter) drives as its front-end -- a build tool, not part of the oracle.
+# Outputs: oracle/_ref/yask/        the reference's own output tree (build products and intermediates);
+#          oracle/_ref/ship/        what the tests and bench.py run, kept apart from that tree so that it can be
+#                                   copied on its own to a machine without the reference:
+#            bin/, lib/             the reference harnesses and drivers of the benchmarked stencils;
+#            refc/                  the reference's stencil COMPILER, which the product's build-time CUDA emitter
+#                                   (yask_b200/emitter) drives as its front-end -- a build tool, not part of the oracle;
+#            tests/                 the reference's own C++ API tests (src/kernel/tests), compiled unmodified against
+#                                   this project's C++ API header and libraries (yask_b200/lib, built first), and its
+#                                   Python API tests, byte-compiled.
 set -e
 REF=${YASK_REFERENCE:-/root/reference}
 HERE=$(cd "$(dirname "$0")" && pwd)
@@ -37,10 +42,15 @@ mkdir -p "$OUT"
 LOG=$HERE/_ref/build.log
 : > "$LOG"
 
-REFC=$(cd "$HERE/.." && pwd)/tools/_refc
+SHIP=$HERE/_ref/ship
+REFC=$SHIP/refc
 if [ ! -x "$REFC/bin/yask_compiler.exe" ]; then
-    echo "[build_ref] yask compiler -> tools/_refc"
+    echo "[build_ref] yask compiler -> oracle/_ref/ship/refc"
     mkdir -p "$REFC"
+    # the library first, with a SONAME: the executable then records it by name, not by this tree's path, so the staged
+    # compiler runs wherever ship/ is copied (the emitter puts refc/lib on LD_LIBRARY_PATH)
+    make -C "$REF/src/compiler" YASK_OUTPUT_DIR="$REFC" mpi=0 arch=$ARCH -j$J EXTRA_YC_CXXFLAGS=-Wl,-soname,libyask_compiler.so \
+        "$REFC/lib/libyask_compiler.so" >> "$LOG" 2>&1
     make -C "$REF/src/compiler" YASK_OUTPUT_DIR="$REFC" mpi=0 arch=$ARCH -j$J compiler >> "$LOG" 2>&1
     rm -rf "$REFC/build"
 fi
@@ -100,14 +110,37 @@ if [ "${REF_ALL:-0}" = "1" ]; then
     done
 fi
 # Strip debug info (the reference builds with -g) and drop the (large) intermediate build tree.
-strip --strip-debug "$OUT"/lib/libyask_kernel.*.so "$OUT"/bin/yask_kernel.*.exe "$OUT"/bin/ref_driver.* 2>/dev/null || true
+strip --strip-debug "$OUT"/lib/libyask_kernel.*.so "$OUT"/bin/yask_kernel.*.exe "$OUT"/bin/ref_driver.* "$REFC"/bin/* "$REFC"/lib/* 2>/dev/null || true
 if [ "${KEEP_BUILD:-0}" != "1" ]; then rm -rf "$OUT/build"; fi
 # what the GPU box runs: the reference harnesses of the three benchmarked stencils and the iso3dfd API drivers
-SHIP=$HERE/_ref/ship
 mkdir -p "$SHIP/bin" "$SHIP/lib"
 for tag in iso3dfd.$ARCH iso3dfd-strict.$ARCH awp_elastic.$ARCH ssg-fp64.$ARCH; do
     [ -f "$OUT/lib/libyask_kernel.$tag.so" ] || continue
     cp -u "$OUT/lib/libyask_kernel.$tag.so" "$SHIP/lib/"
     cp -u "$OUT/bin/yask_kernel.$tag.exe" "$OUT/bin/ref_driver.$tag" "$SHIP/bin/" 2>/dev/null || true
 done
+# the reference's own API tests against this project's libraries, on the solutions those libraries are built for
+# (yask_b200/csrc/Makefile YK_STENCILS); the Python ones run with the pybind11 modules under yask_b200/lib/python
+YB=$(cd "$HERE/.." && pwd)/yask_b200
+TESTS=$REF/src/kernel/tests
+if [ -f "$YB/lib/libyask_b200.so" ]; then
+    mkdir -p "$SHIP/tests"
+    api_test() {    # source  stencil  output
+        local out=$SHIP/tests/$3
+        if [ ! -x "$out" ] || [ "$TESTS/$1.cpp" -nt "$out" ] || [ "$YB/include/yask_kernel_api.hpp" -nt "$out" ]; then
+            g++ -std=c++17 -O1 -I"$YB/include" "$TESTS/$1.cpp" -L"$YB/lib" -lyask_kernel.$2.b200 -lyask_b200 \
+                -Wl,-rpath,'$ORIGIN/../../../../yask_b200/lib' -o "$out"
+        fi
+    }
+    for st in iso3dfd awp_elastic ssg test_3d; do
+        api_test yask_kernel_api_test $st ref_kernel_api_test.$st
+    done
+    api_test yask_kernel_api_exception_test iso3dfd ref_kernel_api_exception_test.iso3dfd
+    for t in yask_kernel_api_test yask_kernel_api_exception_test; do
+        ${PYTHON:-python} -c "import py_compile, sys; py_compile.compile(sys.argv[1], cfile=sys.argv[2], doraise=True)" \
+            "$TESTS/$t.py" "$SHIP/tests/ref_$t.pyc"
+    done
+else
+    echo "[build_ref] yask_b200/lib not built: the reference's API tests are not compiled"
+fi
 echo "[build_ref] done: $(ls "$OUT/bin" | grep -c ref_driver) reference driver(s) under $OUT/bin"

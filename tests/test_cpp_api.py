@@ -4,9 +4,11 @@
   public yk_* API to make the golden fixtures -- compiled unchanged against OUR header and library.  Feeding it the
   fixtures' inputs must reproduce the reference's outputs.
 * `ref_kernel_api_test.<stencil>` / `ref_kernel_api_exception_test` are the reference's own API tests
-  (/root/reference/src/kernel/tests/*.cpp), compiled unmodified against our header in the build container.
+  (src/kernel/tests/*.cpp of the reference), compiled unmodified against our header and libraries by oracle/build_ref.sh
+  into oracle/_ref/ship/tests.
 """
 import os
+import re
 import subprocess
 import tempfile
 
@@ -17,10 +19,11 @@ from tests.helpers import field_ulps, golden_cases, load_golden, regen_inputs
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "tests", "_bin")
+REF_TESTS = os.path.join(ROOT, "oracle", "_ref", "ship", "tests")
 
 
-def _bin(name):
-    p = os.path.join(BIN, name)
+def _bin(name, where=BIN):
+    p = os.path.join(where, name)
     if not os.path.exists(p):
         pytest.skip(f"{name} not built (run __graft_entry__.build())")
     return p
@@ -32,18 +35,20 @@ def test_cpp_api_fails_loudly_without_a_device():
         pytest.skip("a CUDA device is present")
     r = subprocess.run([_bin("yk_driver.iso3dfd"), "info", "32", "32", "32"], capture_output=True, text=True)
     assert r.returncode != 0 and "no CUDA device" in (r.stdout + r.stderr)
-    r = subprocess.run([_bin("ref_kernel_api_exception_test.iso3dfd")], capture_output=True, text=True)
+    r = subprocess.run([_bin("ref_kernel_api_exception_test.iso3dfd", REF_TESTS)], capture_output=True, text=True)
     # first expected exception (run before prepare) is raised with the reference's message
     assert "run_solution() called without calling prepare_solution() first" in r.stdout + r.stderr
 
 
-def _drive(stencil, n, steps, ins, opts=()):
+def _drive(stencil, n, steps, ins, radius=None):
     exe = _bin(f"yk_driver.{stencil}")
+    # the library's radius is fixed by its name; YASK_B200_RADIUS overrides it like the reference's `make radius=<r>`
+    env = dict(os.environ, YASK_B200_RADIUS=str(radius)) if radius else None
     with tempfile.TemporaryDirectory() as d:
         for (name, t), a in ins.items():
             np.ascontiguousarray(a).tofile(os.path.join(d, f"{name}.t{t}.in"))
         n3 = list(n) + [1] * (3 - len(n))
-        r = subprocess.run([exe, "run"] + [str(i) for i in n3] + [str(steps), d], capture_output=True, text=True)
+        r = subprocess.run([exe, "run"] + [str(i) for i in n3] + [str(steps), d], capture_output=True, text=True, env=env)
         assert r.returncode == 0, r.stdout + r.stderr
         outs = {}
         for fn in os.listdir(d):
@@ -67,7 +72,8 @@ def _driver_cases():
 def test_same_driver_source_reproduces_reference_outputs(path):
     meta, arrays = load_golden(path)
     ins = regen_inputs(meta)
-    outs = _drive(meta["stencil"], meta["n"], meta["steps"], ins)
+    radius = re.search(r"-r(\d+)[-.]", meta["ref_tag"])          # iso3dfd fixtures of the reference built at another radius
+    outs = _drive(meta["stencil"], meta["n"], meta["steps"], ins, radius=radius and int(radius.group(1)))
     for key, ref in arrays.items():
         got = outs[key].reshape(ref.shape)
         if meta["stencil"] == "iso3dfd":
@@ -81,14 +87,14 @@ def test_same_driver_source_reproduces_reference_outputs(path):
 @pytest.mark.gpu
 @pytest.mark.parametrize("stencil", ["test_3d", "iso3dfd", "awp_elastic", "ssg"])   # the reference runs it on test_3d
 def test_reference_kernel_api_test_passes_unmodified(stencil):
-    r = subprocess.run([_bin(f"ref_kernel_api_test.{stencil}")], capture_output=True, text=True, timeout=300)
+    r = subprocess.run([_bin(f"ref_kernel_api_test.{stencil}", REF_TESTS)], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout[-3000:], r.stderr[-2000:])
     assert "End of YASK C++ kernel API test." in r.stdout
 
 
 @pytest.mark.gpu
 def test_reference_kernel_api_exception_test_passes_unmodified():
-    r = subprocess.run([_bin("ref_kernel_api_exception_test.iso3dfd")], capture_output=True, text=True, timeout=300)
+    r = subprocess.run([_bin("ref_kernel_api_exception_test.iso3dfd", REF_TESTS)], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout[-3000:], r.stderr[-2000:])
 
 

@@ -1,5 +1,6 @@
 """The CUDA emitter (yask_b200/emitter/yask_cuda_emit.py) re-run on the reference compiler's output must reproduce the
-committed generated sources (kernels + oracle restatement) -- build container only (needs tools/_refc/bin/yask_compiler.exe, built by oracle/build_ref.sh);
+committed generated sources (kernels + oracle restatement) -- needs the reference's compiler, which oracle/build_ref.sh stages
+under oracle/_ref/ship/refc;
 plus parser unit checks that need no reference."""
 import json
 import os
@@ -19,7 +20,7 @@ MAN = json.load(open(os.path.join(GEN, "manifest.json")))
                                   "test_reverse_2d", "iso3dfd_sponge", "wave2d"])
 def test_emitter_reproduces_committed_sources(name):
     if not os.path.exists(E.COMPILER):
-        pytest.skip("reference compiler not built (oracle/build_ref.sh; build container only)")
+        pytest.skip("reference compiler not built (oracle/build_ref.sh)")
     m = MAN[name]
     text = E.run_frontend(m["stencil"], m["elem_bytes"], m.get("radius") or None)
     ir = E.parse_generated(text, name)

@@ -5,11 +5,15 @@
     for the direct kernel, every FP mode, every tile shape of the TMA kernel),
   * TMA kernel vs direct kernel on the device at sizes the oracle cannot reach (checksum equality).
 """
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.helpers import contract_mode_of, golden_cases, load_golden, regen_inputs
+from tests.helpers import GOLDEN, contract_mode_of, golden_cases, load_golden, regen_inputs
 from yask_b200 import capi
 from yask_b200.synth import hash_field, var_salt
 
@@ -219,22 +223,18 @@ def test_tma_equals_direct_on_device_large(n, steps):
 @pytest.mark.parametrize("tag,fp_mode", [("iso3dfd.avx512", 2), ("iso3dfd-strict.avx512", 0)])
 @pytest.mark.parametrize("steps", [1, 2, 10])
 def test_config1_live_reference_128(tag, fp_mode, steps):
-    """BASELINE.json config 1 as written: iso3dfd order 16 fp32 128^3, one rank, against the UNMODIFIED reference run live
-    on this box's CPU (oracle/_ref/ship, built by oracle/build_ref.sh from /root/reference) on identical inputs, bit for bit
-    (the default build against fp_mode 2, the -ffp-contract=off build against fp_mode 0)."""
-    if not O.ref_available(tag):
-        pytest.skip(f"prebuilt reference driver {tag} not present")
-    if "avx512f" not in open("/proc/cpuinfo").read():
-        pytest.skip("host CPU lacks AVX-512")
+    """BASELINE.json config 1 as written: iso3dfd order 16 fp32 128^3, one rank, against the UNMODIFIED reference on
+    identical inputs, bit for bit (the default build against fp_mode 2, the -ffp-contract=off build against fp_mode 0).
+    The reference's outputs are stored as the SHA-256 of their bytes and a seeded sample of points
+    (tests/golden/iso3dfd_config1_128.json, written by `tests/golden/make_golden.py config1`)."""
+    ref = json.load(open(os.path.join(GOLDEN, "iso3dfd_config1_128.json")))[f"{tag}/{steps}"]
     n = (128, 128, 128)
     ins = synth_inputs(n, 1234)
-    outs, after = O.ref_run(tag, n, steps, {("p", 0): ins[("p", 0)], ("p", 1): ins[("p", 1)], ("v", 0): ins[("v", 0)]})
-    tl = after["vars"]["p"]["steps"][1]
-    ref = outs[("p", tl)]
     for kernel in ("tma", "direct"):
         got = run_gpu(n, steps, ins, fp_mode=fp_mode, opts={"kernel": kernel})
-        assert got.shape == ref.shape
-        assert np.array_equal(got.view(np.uint32), ref.view(np.uint32)), kernel
+        assert list(got.shape) == ref["shape"]
+        assert got.view(np.uint32).ravel()[ref["index"]].tolist() == ref["bits"], kernel
+        assert hashlib.sha256(np.ascontiguousarray(got).tobytes()).hexdigest() == ref["sha256"], kernel
 
 
 def test_fuse_vars_shares_storage_between_solutions():

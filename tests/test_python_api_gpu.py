@@ -1,5 +1,6 @@
-"""The reference's own Python API tests, UNMODIFIED (/root/reference/src/kernel/tests/yask_kernel_api_test.py and
-yask_kernel_api_exception_test.py, byte-compiled by the build into tests/_bin like the compiled C++ API tests), run against the
+"""The reference's own Python API tests, UNMODIFIED (src/kernel/tests/yask_kernel_api_test.py and
+yask_kernel_api_exception_test.py of the reference, byte-compiled by oracle/build_ref.sh into oracle/_ref/ship/tests next to
+the compiled C++ API tests), run against the
 `yask_kernel` module of this engine (pybind11, yask_b200/csrc/yk_pybind.cpp) on the GPU: vars are filled through NumPy
 buffers, read back, the solution runs 1 + 4 steps, stats are read -- every assert in those scripts must hold."""
 import glob
@@ -12,14 +13,14 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "tests", "_bin")
+BIN = os.path.join(ROOT, "oracle", "_ref", "ship", "tests")
 MODS = sorted(glob.glob(os.path.join(ROOT, "yask_b200", "lib", "python", "*", "yask_kernel*.so")))
 
 
 def _run(script, mod):
     path = os.path.join(BIN, script)
     if not os.path.exists(path):
-        pytest.skip(f"{script} was not built (outside the container that holds the reference)")
+        pytest.skip(f"{script} was not built (oracle/build_ref.sh)")
     env = dict(os.environ, PYTHONPATH=os.path.dirname(mod))
     return subprocess.run([sys.executable, path], env=env, capture_output=True, text=True, timeout=600)
 

@@ -35,10 +35,11 @@ import sys
 import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-# The reference's stencil compiler, built out of tree from the unmodified sources by oracle/build_ref.sh into tools/_refc
-# (build container only; the emitter's outputs are committed, nothing at run time needs it).
-COMPILER = os.path.join(ROOT, "tools", "_refc", "bin", "yask_compiler.exe")
-COMPILER_LIB = os.path.join(ROOT, "tools", "_refc", "lib")
+# The reference's stencil compiler, built out of tree from the unmodified sources by oracle/build_ref.sh into
+# oracle/_ref/ship/refc (the emitter's outputs are committed, nothing at run time needs it).
+REFC = os.path.join(ROOT, "oracle", "_ref", "ship", "refc")
+COMPILER = os.path.join(REFC, "bin", "yask_compiler.exe")
+COMPILER_LIB = os.path.join(REFC, "lib")
 
 
 class EmitError(RuntimeError):
@@ -56,7 +57,7 @@ def c_ident(name: str) -> str:
 # ----------------------------------------------------------------------------------------------------
 def run_frontend(stencil: str, elem_bytes: int, radius: int | None) -> str:
     if not os.path.exists(COMPILER):
-        raise EmitError(f"{COMPILER} missing: run oracle/build_ref.sh first (build container only)")
+        raise EmitError(f"{COMPILER} missing: run oracle/build_ref.sh first (needs the reference's sources)")
     with tempfile.TemporaryDirectory() as d:
         out = os.path.join(d, "gen.hpp")
         cmd = [COMPILER, "-stencil", stencil, "-target", "avx512", "-elem-bytes", str(elem_bytes), "-p", out]
